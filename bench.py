@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- motions/sec of the MDM sampling hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c2|c3|dip|a2m]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c2|c3|dip|a2m] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one complete sampling loop over one batch.  Default (--config c2) = BASELINE config 2 -- HumanML3D shapes,
@@ -18,6 +18,10 @@ Other BASELINE configs (same JSON line, their own FLOP count from SURVEY.md sect
   roofline     : the dominant kernel of the step (see DESIGN.md section 4) timed alone with CUDA events, L2 flushed
   cpu_baseline : the reference's own CPU p_sample_loop (unmodified files in oracle/_ref, kind "reference") on a bounded
                  sample: full 50 steps, as many of the 64 motions as the time box allows; the oracle port if _ref is absent
+--dump-outputs DIR writes DIR/sample.npy (float32): the motions the last timed resident loop returned to its caller (rank
+0's shard with several GPUs).  Weights, conditioning and noise come from fixed seeds (torch's default generators, which
+DiP draws its noise from, are seeded per rank at start-up), so two builds run with the same arguments can be compared
+output for output.
 Multi-GPU: batch sharded, one NCCL broadcast of the text embedding per loop, nothing inside the loop ("weak" scaling:
 64 motions per GPU).
 """
@@ -519,7 +523,13 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the sample the last timed step returned as DIR/sample.npy (float32)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs the GPU path (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -530,6 +540,7 @@ def main():
     import torch.distributed as dist
     assert torch.cuda.is_available(), "bench.py needs a B200"
     torch.cuda.set_device(local)
+    torch.manual_seed(7 + rank)   # the paths that draw from torch's default generators (DiP, e2e) start from a fixed state
     dev = torch.device("cuda", local)
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
@@ -539,13 +550,15 @@ def main():
     eng, one_loop_resident, one_loop_e2e, h2d, d2h, l2_note = build_workload(a.config, B, rank, world, dev)
 
     def timed(fn, iters):
+        """Milliseconds of `iters` calls of fn between two CUDA events, and what the last call returned."""
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(iters):
-            fn()
+        for _ in range(iters - 1):
+            fn()                  # results dropped at once, as in the warm-up: the allocator reuses one output block
+        last = fn()
         e1.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -553,7 +566,7 @@ def main():
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), last
 
     def log(msg):
         if rank == 0:
@@ -575,7 +588,7 @@ def main():
             sampler.start()
         except Exception as e:   # noqa: BLE001
             sampler.errors.append("start: %r" % (e,))
-    ms_total = timed(one_loop_resident, a.steps)
+    ms_total, last_sample = timed(one_loop_resident, a.steps)
     try:
         clocks = sampler.stop() if rank == 0 else None
     except Exception as e:   # noqa: BLE001
@@ -585,7 +598,7 @@ def main():
     log("resident loops timed: %.2f ms per loop" % (ms_total / a.steps))
     for _ in range(2):
         one_loop_e2e()
-    ms_e2e = timed(one_loop_e2e, a.steps)
+    ms_e2e, _ = timed(one_loop_e2e, a.steps)
     log("e2e loops timed: %.2f ms per loop" % (ms_e2e / a.steps))
 
     ms_step = ms_total / a.steps
@@ -631,6 +644,12 @@ def main():
                 "roofline": roof, "cpu_baseline": cpu,
                 "flop_per_motion": cfg["flop_per_motion"]}
         print(json.dumps(line), flush=True)
+        if a.dump_outputs:
+            import numpy as np
+            os.makedirs(a.dump_outputs, exist_ok=True)
+            path = os.path.join(a.dump_outputs, "sample.npy")
+            np.save(path, last_sample.float().cpu().numpy())
+            log("last timed sample %s -> %s" % (tuple(last_sample.shape), path))
     if world > 1:
         dist.destroy_process_group()
 

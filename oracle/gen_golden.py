@@ -12,8 +12,10 @@ Files
                  space_timesteps known answers (sorted lists) incl. the ValueError case
   enc_small.npz  trans_enc L=2, B=3, T=24, 4 steps, ragged lengths, per-sample scales: single forwards (cond,
                  uncond, CFG), every p_sample output of p_sample_loop, ddim (eta 0 and 0.5) loop outputs,
-                 inpainting loop output, skip_timesteps/init_image output
+                 inpainting loop output, skip_timesteps/init_image output (the motion they start from is not stored:
+                 tests/conftest.py inpaint_motion() draws it from the same seed, which keeps the file under 1 MB)
   enc_c1.npz     BASELINE config 1 shape: L=8, B=1, T=196, 50 steps, CFG 2.5 -> final sample
+  enc_l3.npz     trans_enc L=3, B=2, T=31, 6 steps on seeds of its own: final sample, timestep map, diffusion tables
   a2m_small.npz  action-conditioned trans_enc (humanact12 shape 25x6, 12 classes), no CFG, 3 steps
   ric.npz        post-loop inv_transform + recover_from_ric (generate.py:161-166), 263- and 251-dim features
   dip_small.npz  trans_dec + BERT-token memory + prefix completion (DiP): L=2, ctx 20 + pred 40, 3 steps, ragged text
@@ -32,16 +34,16 @@ from oracle import ref_harness as rh  # noqa: E402
 
 syn = importlib.import_module("motion-diffusion-model_b200.synthetic")
 OUT = os.path.join(ROOT, "tests", "golden")
+TABLE_NAMES = ["betas", "alphas_cumprod", "alphas_cumprod_prev", "alphas_cumprod_next", "sqrt_alphas_cumprod",
+               "sqrt_one_minus_alphas_cumprod", "log_one_minus_alphas_cumprod", "sqrt_recip_alphas_cumprod",
+               "sqrt_recipm1_alphas_cumprod", "posterior_variance", "posterior_log_variance_clipped",
+               "posterior_mean_coef1", "posterior_mean_coef2"]
 
 
 def gen_schedule():
     ns = rh.load_reference()
     gd, rs = ns.gaussian_diffusion, ns.respace
     out = {}
-    names = ["betas", "alphas_cumprod", "alphas_cumprod_prev", "alphas_cumprod_next", "sqrt_alphas_cumprod",
-             "sqrt_one_minus_alphas_cumprod", "log_one_minus_alphas_cumprod", "sqrt_recip_alphas_cumprod",
-             "sqrt_recipm1_alphas_cumprod", "posterior_variance", "posterior_log_variance_clipped",
-             "posterior_mean_coef1", "posterior_mean_coef2"]
     cases = [("cosine", 50, [50]), ("cosine", 1000, [1000]), ("cosine", 1000, "50"), ("cosine", 1000, "ddim50"),
              ("cosine", 10, [10]), ("linear", 1000, "10,15,20"), ("cosine", 300, [10, 15, 20])]
     for ci, (sched, steps, resp) in enumerate(cases):
@@ -52,7 +54,7 @@ def gen_schedule():
         out["case%d_meta" % ci] = np.array([sched, str(steps), repr(resp)])
         out["case%d_base_betas" % ci] = betas
         out["case%d_timestep_map" % ci] = np.array(d.timestep_map, dtype=np.int64)
-        for n in names:
+        for n in TABLE_NAMES:
             out["case%d_%s" % (ci, n)] = getattr(d, n)
     kats = [(300, [10, 15, 20]), (1000, "ddim50"), (1000, "50"), (1000, "ddim25"), (50, [50]), (1000, "10,15,20"),
             (1000, [1]), (7, [3, 2]), (100, "ddim10"), (100, [100])]
@@ -126,7 +128,6 @@ def gen_enc_small():
         yi["inpainting_mask"], yi["inpainted_motion"] = imask, motion
         with rh.noise_tape(inp["tape"]):
             out["ddpm_inpaint"] = diff.p_sample_loop(cfg, shape, clip_denoised=False, model_kwargs={"y": yi}).numpy()
-        out["inpaint_motion"] = motion.numpy()
         # skip_timesteps + init_image (q_sample at the first index)
         with rh.noise_tape(inp["tape"]):
             out["ddpm_skip1_init"] = diff.p_sample_loop(cfg, shape, clip_denoised=False, skip_timesteps=1,
@@ -152,6 +153,25 @@ def gen_enc_c1():
     np.savez_compressed(os.path.join(OUT, "enc_c1.npz"), sample=ref.numpy(),
                         meta=np.array(["L=8 steps=50 B=1 T=196 weights_seed=0 inputs_seed=10 scale=2.5"]))
     print("enc_c1.npz:", tuple(ref.shape), float(ref.abs().mean()))
+
+
+def gen_enc_l3():
+    """A third trans_enc setting on seeds no other fixture uses: L=3, 6 steps, B=2, T=31, ragged lengths, per-sample
+    scales; the final sample, the timestep map and the diffusion tables of the reference."""
+    ns = rh.load_reference()
+    L, steps, B, T = 3, 6, 2, 31
+    sd = syn.synthetic_state_dict(num_layers=L, seed=7)
+    model, diff = rh.build(rh.default_args(layers=L, diffusion_steps=steps), state_dict=sd)
+    cfg = ns.sampler_util.ClassifierFreeSampleModel(model)
+    inp = syn.synthetic_inputs(B, nframes=T, steps=steps, seed=21, lengths=[31, 9], scale=torch.tensor([3.0, 0.5]))
+    with torch.no_grad(), rh.noise_tape(inp["tape"]):
+        ref = diff.p_sample_loop(cfg, (B, 263, 1, T), clip_denoised=False, model_kwargs={"y": _y(inp)})
+    out = {"meta": np.array(["L=3 steps=6 B=2 T=31 weights_seed=7 inputs_seed=21 lengths=31,9 scales=3,0.5"]),
+           "sample": ref.numpy(), "timestep_map": np.array(diff.timestep_map, dtype=np.int64)}
+    for n in TABLE_NAMES:
+        out["table_" + n] = getattr(diff, n)
+    np.savez_compressed(os.path.join(OUT, "enc_l3.npz"), **out)
+    print("enc_l3.npz:", tuple(ref.shape))
 
 
 def gen_a2m_small():
@@ -219,6 +239,7 @@ if __name__ == "__main__":
     gen_schedule()
     gen_enc_small()
     gen_enc_c1()
+    gen_enc_l3()
     gen_a2m_small()
     gen_dip_small()
     gen_ric()

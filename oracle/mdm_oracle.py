@@ -12,8 +12,8 @@ What is restated (paths relative to /root/reference):
   * p_sample_loop(_progressive) ................. diffusion/gaussian_diffusion.py:591-727
 
 Layout: batch-major [B, S, d]; the cond/uncond CFG pair is evaluated as two halves of one batch.
-Pinned against the live reference in tests/test_oracle_cpu.py::test_oracle_vs_live_reference (build
-container) and by tests/golden/*.npz produced by oracle/gen_golden.py from the reference itself.
+Pinned by tests/golden/*.npz, produced by oracle/gen_golden.py from the reference itself
+(tests/test_oracle_cpu.py).
 
 `cast` (optional) rounds both GEMM operands through a narrower dtype and back; it exists only for
 the precision studies behind DESIGN.md section 2 and is None for parity work.

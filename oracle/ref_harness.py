@@ -1,10 +1,9 @@
 """TEST INFRASTRUCTURE ONLY -- never imported by the product path.
 
-Loads the UNMODIFIED reference (GuyTevet/motion-diffusion-model, mounted read-only at
-/root/reference) on CPU so that it can be used as the parity oracle and as the generator of
-the golden vectors under tests/golden/.  /root/reference exists only in the build container;
-nothing that runs on the GPU box may import this module (tests that need it are skipped when
-the directory is absent).
+Loads the UNMODIFIED reference (GuyTevet/motion-diffusion-model) on CPU: oracle/gen_golden.py runs
+it to write the golden vectors under tests/golden/, oracle/build_ref.py to list its hot-path files,
+and bench.py's CPU reference arm to time it.  No test imports this module; the tests compare
+against the stored vectors.
 
 Two third-party imports of the reference are absent here and are stubbed *before* import
 (SURVEY.md section 8c): `clip` (model/mdm.py:5) and `model.rotation2xyz` -> smplx

@@ -2,8 +2,8 @@
 logic.  Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline leg may import this.
 
 Pinned against (a) the known-answer constants probed from the reference (SURVEY.md section 8a rows
-a1-a4) and (b) the live reference in the build container (tests/test_oracle_vs_reference.py) and
-(c) tests/golden/schedule_*.npz written by oracle/gen_golden.py from the reference itself.
+a1-a4) and (b) the tables in tests/golden/schedule.npz and enc_l3.npz, written by oracle/gen_golden.py from the
+reference itself.
 
 Each function cites the reference lines it restates (paths relative to /root/reference).
 """

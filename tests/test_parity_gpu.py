@@ -11,7 +11,7 @@ import pytest
 import torch
 
 import b200mdm
-from conftest import default_args, rel_err
+from conftest import default_args, inpaint_motion, rel_err
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-3
@@ -87,7 +87,7 @@ def test_loop_variants_vs_reference_golden(golden):
         o = diffusion.ddim_sample_loop(cfg, shape, noise=xT, clip_denoised=False, eta=eta, model_kwargs={"y": _y(inp)},
                                        noise_tape=tape)
         assert rel_err(o, g["ddim_eta%g" % eta]) < RTOL, eta
-    motion = torch.from_numpy(g["inpaint_motion"]).cuda()
+    motion = inpaint_motion().cuda()
     m = torch.zeros(shape, dtype=torch.bool, device="cuda")
     m[..., :8] = True
     yi = _y(inp)
