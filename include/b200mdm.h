@@ -49,6 +49,11 @@ extern "C" {
 #define B200MDM_FLAG_PHILOX_NOISE 4  /* loops only: eps comes from the engine's counter-based stream (b200mdm_set_noise_stream)
                                         instead of a caller-provided tape -- replaces th.randn_like, gaussian_diffusion.py:525 */
 
+#define B200MDM_TARGET_NONE 0
+#define B200MDM_TARGET_SINGLE 1 /* EmbedTargetLocSingle (model/mdm.py:399-419) */
+#define B200MDM_TARGET_MULTI 2  /* EmbedTargetLocMulti  (model/mdm.py:449-480) */
+#define B200MDM_TARGET_SPLIT 3  /* EmbedTargetLocSplit  (model/mdm.py:422-447) */
+
 #define B200MDM_SCHED_STRIDE 8 /* floats per schedule row, see b200mdm_set_schedule */
 
 typedef struct b200mdm_engine b200mdm_engine;
@@ -70,7 +75,13 @@ typedef struct b200mdm_config {
   int32_t pos_embed_max_len; /* args.pos_embed_max_len: rows of the positional table */
   int32_t temb_rows;         /* model timesteps to pre-embed (>= original_num_steps of the diffusion) */
   int32_t context_len;       /* trans_dec (DiP) prefix completion: args.context_len frames precede x (model/mdm.py:58-61) */
-  int32_t reserved[6];
+  /* target-location conditioning (args.multi_target_cond, model/mdm.py:64-73): B200MDM_TARGET_*; 0 = the model has no
+   * embed_target_cond.  n_goal_rows = len(all_goal_joint_names) + 2 ('traj', 'heading'; 8 for humanml), and
+   * target_enc_layers = args.target_enc_layers (single / split encoders; the multi encoder has a fixed depth). */
+  int32_t target_encoder;
+  int32_t n_goal_rows;
+  int32_t target_enc_layers;
+  int32_t reserved[3];
 } b200mdm_config;
 
 const char* b200mdm_last_error(void);
@@ -81,13 +92,17 @@ int b200mdm_create(const b200mdm_config* cfg, b200mdm_engine** out);
 int b200mdm_destroy(b200mdm_engine* e);
 
 /* load_model_wo_clip / load_state_dict(strict=False) (utils/model_util.py:8-15): one call per state_dict entry,
- * `name` is the reference key (SURVEY.md A.4), data fp32, host or device memory.  "sequence_pos_encoder.pe"
+ * `name` is the reference key (SURVEY.md A.4), data fp32, host or device memory.  The target encoder's keys are the
+ * reference's embed_target_cond.* names, except that the multi encoder's per-joint MLPs are addressed by row index:
+ * embed_target_cond.target_loc_emb.<row>.{0,2}.{weight,bias} (row = position in all_goal_joint_names + ['traj',
+ * 'heading']; the reference keys them by joint name).  "sequence_pos_encoder.pe"
  * ([max_len, d]; the buffer the reference recomputes in PositionalEncoding.__init__, model/mdm.py:301-308) is
  * accepted here as well.  Unknown names -> B200MDM_EINVAL (the reference asserts no unexpected keys). */
 int b200mdm_load_weight(b200mdm_engine* e, const char* name, const float* data, const int64_t* shape, int32_t ndim);
 
 /* Repack for the tensor cores (fp16 K-major copies, hi/lo split of the in/out projections), precompute the
- * timestep-embedding MLP (TimestepEmbedder.forward, model/mdm.py:329-330) for every model timestep.
+ * timestep-embedding MLP (TimestepEmbedder.forward, model/mdm.py:329-330) for every model timestep and the normalised
+ * row weights of the multi target encoder (WeightedSum, utils/misc.py:12).
  * Fails with B200MDM_ESTATE listing the first missing tensor. */
 int b200mdm_finalize_weights(b200mdm_engine* e, void* stream);
 
@@ -120,6 +135,18 @@ int b200mdm_set_cond(b200mdm_engine* e, int32_t batch, int32_t nframes, const fl
 int b200mdm_set_cond_dec(b200mdm_engine* e, int32_t batch, int32_t nframes, const float* enc_text_dev,
                          const uint8_t* text_mask_host, int32_t n_tokens, const int64_t* lengths_host,
                          const float* scale_dev, int32_t force_uncond, void* stream);
+/* Target-location conditioning (model/mdm.py:197-199): embed_target_cond(y['target_cond'], y['target_joint_names'],
+ * y['is_heading']) for an engine created with target_encoder != 0.  The embedding does not depend on the timestep, so it is
+ * computed here, once per loop, into an engine-owned buffer, and the NEXT b200mdm_set_cond / b200mdm_set_cond_dec adds it
+ * to every conditioning row it builds (trans_enc: the conditioning token; DiP: every row of the cross-attention memory),
+ * in both halves of a CFG pair and after the text masking of `uncond` (the reference adds it to time_emb, which both
+ * halves share).  The step graph and its launches are unchanged.
+ *   target_cond_dev : y['target_cond'] fp32 [batch, n_goal_rows, 3] device; NULL clears the target (no 'target_cond' key,
+ *                     or y['target_uncond']: mask_cond zeros the embedding), giving exactly the computation without targets
+ *   valid_host      : uint8 [batch, n_goal_rows], 1 where the row's name is in target_joint_names[b] (row
+ *                     n_goal_rows - 1, 'heading', when is_heading[b])
+ * The target is consumed by the next set_cond*, which fails with B200MDM_EINVAL if its batch differs from `batch`. */
+int b200mdm_set_target(b200mdm_engine* e, int32_t batch, const float* target_cond_dev, const uint8_t* valid_host, void* stream);
 /* y['prefix'] [batch, njoints, nfeats, context_len] fp32 device: the frames x is a continuation of. */
 int b200mdm_set_prefix(b200mdm_engine* e, const float* prefix_dev, void* stream);
 

@@ -14,7 +14,8 @@ from .utils.sampler_util import ClassifierFreeSampleModel, AutoRegressiveSampler
 from .diffusion.respace import SpacedDiffusion, space_timesteps  # noqa: F401
 from .diffusion.gaussian_diffusion import GaussianDiffusion, get_named_beta_schedule  # noqa: F401
 from .model.mdm import MDM  # noqa: F401
-from .synthetic import synthetic_state_dict, synthetic_inputs, synthetic_dip_inputs, synthetic_norm_stats  # noqa: F401
+from .synthetic import (synthetic_state_dict, synthetic_inputs, synthetic_dip_inputs, synthetic_norm_stats,  # noqa: F401
+                        synthetic_targets)
 
 __version__ = "0.1.0"
 from .data_loaders.humanml.scripts.motion_process import recover_from_ric, sample_to_xyz  # noqa: F401,E402

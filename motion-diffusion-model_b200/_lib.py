@@ -12,6 +12,7 @@ OK, EINVAL, ECUDA, ESTATE, ENOTIMPL = 0, -1, -2, -3, -4
 ARCH = {"trans_enc": 0, "trans_dec": 1}
 COND_NONE, COND_TEXT, COND_ACTION = 0, 1, 2
 MODE_X0, MODE_DDPM, MODE_DDIM = 0, 1, 2
+TARGET = {None: 0, "single": 1, "multi": 2, "split": 3}
 FLAG_CONST_NOISE, FLAG_CLIP_DENOISED, FLAG_PHILOX_NOISE = 1, 2, 4
 SCHED_STRIDE = 8
 
@@ -19,7 +20,7 @@ SCHED_STRIDE = 8
 SYMBOLS = [
     "b200mdm_last_error", "b200mdm_version", "b200mdm_create", "b200mdm_destroy", "b200mdm_load_weight",
     "b200mdm_finalize_weights", "b200mdm_set_schedule", "b200mdm_set_cond", "b200mdm_set_cond_dec", "b200mdm_set_prefix",
-    "b200mdm_set_inpaint",
+    "b200mdm_set_inpaint", "b200mdm_set_target",
     "b200mdm_denoise", "b200mdm_sample_step", "b200mdm_sample_loop", "b200mdm_q_sample", "b200mdm_launch_count",
     "b200mdm_sample_loop_range", "b200mdm_set_noise_stream", "b200mdm_philox_normal",
     "b200mdm_recover_from_ric", "b200mdm_test_gemm_f16", "b200mdm_test_attention", "b200mdm_test_cross_attention", "b200mdm_test_qkv_attention", "b200mdm_test_gemm_resid_ln",
@@ -30,7 +31,8 @@ SYMBOLS = [
 class Config(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in (
         "arch", "latent_dim", "ff_size", "num_layers", "num_heads", "njoints", "nfeats", "cond_mode", "cond_dim",
-        "num_actions", "mask_frames", "pos_embed_max_len", "temb_rows", "context_len")] + [("reserved", ctypes.c_int32 * 6)]
+        "num_actions", "mask_frames", "pos_embed_max_len", "temb_rows", "context_len", "target_encoder", "n_goal_rows",
+        "target_enc_layers")] + [("reserved", ctypes.c_int32 * 3)]
 
 
 class B200MDMError(RuntimeError):
@@ -65,6 +67,8 @@ def load():
     lib.b200mdm_set_cond.argtypes = [vp, i32, i32, vp, vp, vp, i32, vp, vp]
     lib.b200mdm_set_cond_dec.argtypes = [vp, i32, i32, vp, vp, i32, vp, vp, i32, vp]
     lib.b200mdm_set_prefix.argtypes = [vp, vp, vp]
+    if hasattr(lib, "b200mdm_set_target"):           # (absent from A/B builds that predate target conditioning)
+        lib.b200mdm_set_target.argtypes = [vp, i32, vp, vp, vp]
     lib.b200mdm_set_inpaint.argtypes = [vp, vp, vp]
     lib.b200mdm_recover_from_ric.argtypes = [vp, i64, i64, i64, vp, vp, vp, i64, i64, i64, i32, i32, i32, vp]
     lib.b200mdm_denoise.argtypes = [vp, vp, vp, vp, vp]

@@ -25,6 +25,7 @@
 #include "postprocess.cuh"
 #include "qkv_attn.cuh"
 #include "kernels.cuh"
+#include "target_embed.cuh"
 
 using namespace b200;
 
@@ -216,6 +217,15 @@ struct b200mdm_engine : Workspace {
   cudaStream_t work = nullptr;
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;
   long long launches = 0;
+  // target-location encoder (b200mdm_set_target): weights packed per stage as [groups, N, K] / [groups, N], buffers sized
+  // for `tgt_cap` samples (they only grow), and the embedding the next set_cond* folds into its conditioning rows
+  std::vector<float*> tgt_w, tgt_b;
+  float* tgt_wn = nullptr;                                   // multi: w / sum(w)
+  float *tgt_out = nullptr, *tgt_ha = nullptr, *tgt_hb = nullptr, *tgt_x0 = nullptr;
+  int* tgt_idx = nullptr;                                    // [n counts | n x cap sample lists | cap x n validity]
+  int tgt_cap = 0, tgt_batch = 0;
+  bool tgt_pending = false;
+  std::vector<int> h_tgt;
 };
 
 template <class T>
@@ -464,6 +474,17 @@ extern "C" int b200mdm_create(const b200mdm_config* cfg, b200mdm_engine** out) {
                 cfg->num_heads);
   if (cfg->num_layers <= 0 || cfg->njoints <= 0 || cfg->nfeats <= 0 || cfg->pos_embed_max_len <= 0 || cfg->temb_rows <= 0)
     return fail(B200MDM_EINVAL, "bad config");
+  if (cfg->target_encoder != B200MDM_TARGET_NONE) {
+    if (cfg->target_encoder < B200MDM_TARGET_SINGLE || cfg->target_encoder > B200MDM_TARGET_SPLIT)
+      return fail(B200MDM_ENOTIMPL, "target_encoder %d: single (1), multi (2) and split (3) are implemented", cfg->target_encoder);
+    if (cfg->n_goal_rows < 1 || cfg->n_goal_rows > 64)
+      return fail(B200MDM_ENOTIMPL, "target encoder: n_goal_rows %d outside 1..64", cfg->n_goal_rows);
+    if (cfg->target_encoder != B200MDM_TARGET_MULTI && cfg->target_enc_layers < 1)
+      return fail(B200MDM_ENOTIMPL, "target encoder: target_enc_layers %d (>= 1 implemented)", cfg->target_enc_layers);
+    if (cfg->target_encoder == B200MDM_TARGET_SPLIT && cfg->latent_dim % cfg->n_goal_rows)
+      return fail(B200MDM_ENOTIMPL, "split target encoder needs latent_dim %% n_goal_rows == 0 (%d, %d)", cfg->latent_dim,
+                  cfg->n_goal_rows);
+  }
   int dev = 0;
   CUDA_TRY(cudaGetDevice(&dev));
   cudaDeviceProp prop;
@@ -522,6 +543,19 @@ static void drop_all_graphs(b200mdm_engine* e) {
   for (auto& w : e->pool) drop_graph(&w);
 }
 
+static void free_target(b200mdm_engine* e, bool buffers) {
+  for (float* p : e->tgt_w) cudaFree(p);
+  for (float* p : e->tgt_b) cudaFree(p);
+  e->tgt_w.clear();
+  e->tgt_b.clear();
+  dfree(e->tgt_wn);
+  if (buffers) {
+    dfree(e->tgt_out); dfree(e->tgt_ha); dfree(e->tgt_hb); dfree(e->tgt_x0); dfree(e->tgt_idx);
+    e->tgt_cap = 0;
+  }
+  e->tgt_pending = false;
+}
+
 extern "C" int b200mdm_destroy(b200mdm_engine* e) {
   if (!e) return B200MDM_OK;
   cudaDeviceSynchronize();
@@ -530,6 +564,7 @@ extern "C" int b200mdm_destroy(b200mdm_engine* e) {
   for (auto& l : e->layers) { dfree(l.wqkv); dfree(l.wo); dfree(l.w1); dfree(l.w2); dfree(l.wq_c); dfree(l.wo_c); }
   dfree(e->w_in3); dfree(e->w_out3); dfree(e->temb_hidden); dfree(e->temb_table); dfree(e->sched); dfree(e->tmap);
   dfree(e->wkv_all); dfree(e->bkv_all);
+  free_target(e, true);
   dfree(e->state);
   if (e->work) cudaStreamDestroy(e->work);
   if (e->ev_in) cudaEventDestroy(e->ev_in);
@@ -539,7 +574,48 @@ extern "C" int b200mdm_destroy(b200mdm_engine* e) {
 }
 
 // ------------------------------------------------------------------------------------------------ weights
+// The target encoder as a chain of grouped linear stages (target_embed.cuh): stage s has `groups` matrices [N, K]; the
+// state_dict name of group g's weight is name(s, g) + ".weight", its bias name(s, g) + ".bias".
+struct TgtStage {
+  int groups, N, K;
+};
+static std::vector<TgtStage> target_stages(const b200mdm_config& c) {
+  const int d = c.latent_dim, n = c.n_goal_rows;
+  std::vector<TgtStage> st;
+  if (c.target_encoder == B200MDM_TARGET_SINGLE) {
+    st.push_back({1, d, 4 * n});
+    for (int l = 0; l < c.target_enc_layers; ++l) st.push_back({1, d, d});
+  } else if (c.target_encoder == B200MDM_TARGET_SPLIT) {
+    st.push_back({n, d / n, 4});
+    for (int l = 0; l < c.target_enc_layers; ++l) st.push_back({n, d / n, d / n});
+  } else if (c.target_encoder == B200MDM_TARGET_MULTI) {
+    st.push_back({n, d, 3});
+    st.push_back({n, d, d});
+  }
+  return st;
+}
+static std::string target_stage_name(const b200mdm_config& c, int s, int g) {
+  const std::string p = "embed_target_cond.";
+  if (c.target_encoder == B200MDM_TARGET_SINGLE) return p + "mlp." + std::to_string(2 * s);
+  if (c.target_encoder == B200MDM_TARGET_SPLIT) return p + "mini_mlps." + std::to_string(g) + "." + std::to_string(2 * s);
+  return p + "target_loc_emb." + std::to_string(g) + "." + std::to_string(2 * s);
+}
+static const char* kTargetRowWeights = "embed_target_cond.target_all_loc_emb.weights";
+
+static bool known_target_name(const b200mdm_engine* e, const std::string& n) {
+  if (e->cfg.target_encoder == B200MDM_TARGET_NONE || n.compare(0, 18, "embed_target_cond.") != 0) return false;
+  if (e->cfg.target_encoder == B200MDM_TARGET_MULTI && n == kTargetRowWeights) return true;
+  const std::vector<TgtStage> st = target_stages(e->cfg);
+  for (size_t s = 0; s < st.size(); ++s)
+    for (int g = 0; g < st[s].groups; ++g) {
+      const std::string base = target_stage_name(e->cfg, static_cast<int>(s), g);
+      if (n == base + ".weight" || n == base + ".bias") return true;
+    }
+  return false;
+}
+
 static bool known_weight_name(const b200mdm_engine* e, const std::string& n) {
+  if (known_target_name(e, n)) return true;
   static const char* fixed[] = {"input_process.poseEmbedding.weight", "input_process.poseEmbedding.bias",
                                 "embed_timestep.time_embed.0.weight", "embed_timestep.time_embed.0.bias",
                                 "embed_timestep.time_embed.2.weight", "embed_timestep.time_embed.2.bias",
@@ -611,6 +687,38 @@ static int to_f16_k(const float* src, __half** dst, int N, int K, int kw, cudaSt
   TRY(dalloc(dst, static_cast<size_t>(N) * K * 2));
   f32_to_f16_dup_kernel<<<512, 256, 0, s>>>(src, *dst, N, K);
   CUDA_TRY(cudaGetLastError());
+  return B200MDM_OK;
+}
+
+// Pack every stage of the target encoder into [groups, N, K] / [groups, N] (one grouped launch per stage), and normalise
+// the multi encoder's row weights.
+static int finalize_target(b200mdm_engine* e, cudaStream_t s) {
+  free_target(e, false);
+  if (e->cfg.target_encoder == B200MDM_TARGET_NONE) return B200MDM_OK;
+  const std::vector<TgtStage> st = target_stages(e->cfg);
+  for (size_t k = 0; k < st.size(); ++k) {
+    const TgtStage& g = st[k];
+    float *w = nullptr, *b = nullptr;
+    TRY(dalloc(&w, static_cast<size_t>(g.groups) * g.N * g.K));
+    e->tgt_w.push_back(w);
+    TRY(dalloc(&b, static_cast<size_t>(g.groups) * g.N));
+    e->tgt_b.push_back(b);
+    for (int j = 0; j < g.groups; ++j) {
+      const std::string base = target_stage_name(e->cfg, static_cast<int>(k), j);
+      const float *src_w, *src_b;
+      TRY(need(e, base + ".weight", {g.N, g.K}, &src_w));
+      TRY(need(e, base + ".bias", {g.N}, &src_b));
+      CUDA_TRY(cudaMemcpyAsync(w + static_cast<size_t>(j) * g.N * g.K, src_w, sizeof(float) * g.N * g.K, cudaMemcpyDeviceToDevice, s));
+      CUDA_TRY(cudaMemcpyAsync(b + static_cast<size_t>(j) * g.N, src_b, sizeof(float) * g.N, cudaMemcpyDeviceToDevice, s));
+    }
+  }
+  if (e->cfg.target_encoder == B200MDM_TARGET_MULTI) {
+    const float* rw;
+    TRY(need(e, kTargetRowWeights, {e->cfg.n_goal_rows}, &rw));
+    TRY(dalloc(&e->tgt_wn, e->cfg.n_goal_rows));
+    tgt_normalise_kernel<<<1, 1, 0, s>>>(rw, e->tgt_wn, e->cfg.n_goal_rows);
+    CUDA_TRY(cudaGetLastError());
+  }
   return B200MDM_OK;
 }
 
@@ -718,6 +826,7 @@ extern "C" int b200mdm_finalize_weights(b200mdm_engine* e, void* stream) {
   CUDA_TRY(cudaGetLastError());
   small_linear_kernel<0><<<blocks, 256, 0, s>>>(e->temb_hidden, t2w, t2b, e->temb_table, R, d, d, d);
   CUDA_TRY(cudaGetLastError());
+  TRY(finalize_target(e, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   e->finalized = true;
   return B200MDM_OK;
@@ -867,11 +976,120 @@ static int select_workspace(b200mdm_engine* e, int B, int T, int halves, cudaStr
 }
 
 
+// ---- target-location conditioning (model/mdm.py:197-199; encoders in target_embed.cuh)
+static int launch_tgt_linear(b200mdm_engine* e, const TgtLinear& p, int groups, int max_rows, cudaStream_t s) {
+  tgt_linear_kernel<<<dim3((p.N + TGT_BN - 1) / TGT_BN, (max_rows + TGT_BM - 1) / TGT_BM, groups), TGT_THREADS, 0, s>>>(p);
+  CUDA_TRY(cudaGetLastError());
+  e->launches++;
+  return B200MDM_OK;
+}
+
+extern "C" int b200mdm_set_target(b200mdm_engine* e, int32_t batch, const float* target_cond_dev, const uint8_t* valid_host,
+                                  void* stream) {
+  if (!e) return fail(B200MDM_EINVAL, "null engine");
+  if (e->cfg.target_encoder == B200MDM_TARGET_NONE)
+    return fail(B200MDM_EINVAL, "this engine has no target encoder (created with target_encoder = 0)");
+  e->tgt_pending = false;
+  if (!target_cond_dev) return B200MDM_OK;   // no target / target_uncond: the conditioning rows stay exactly as without
+  if (!e->finalized) return fail(B200MDM_ESTATE, "weights not finalised");
+  if (batch <= 0 || !valid_host) return fail(B200MDM_EINVAL, "bad batch / null validity mask");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int d = e->d, n = e->cfg.n_goal_rows, B = batch, type = e->cfg.target_encoder;
+  const int hcols = type == B200MDM_TARGET_MULTI ? n * d : d;   // per-sample width of the hidden buffers
+  if (B > e->tgt_cap) {
+    CUDA_TRY(cudaDeviceSynchronize());   // a set_cond* of an earlier loop may still read the old buffer
+    dfree(e->tgt_out); dfree(e->tgt_ha); dfree(e->tgt_hb); dfree(e->tgt_x0); dfree(e->tgt_idx);
+    e->tgt_cap = 0;
+    TRY(dalloc(&e->tgt_out, static_cast<size_t>(B) * d));
+    TRY(dalloc(&e->tgt_ha, static_cast<size_t>(B) * hcols));
+    TRY(dalloc(&e->tgt_hb, static_cast<size_t>(B) * hcols));
+    TRY(dalloc(&e->tgt_x0, static_cast<size_t>(B) * 4 * n));
+    TRY(dalloc(&e->tgt_idx, static_cast<size_t>(n) + 2 * static_cast<size_t>(n) * B));
+    e->tgt_cap = B;
+  }
+  // host staging: per-row sample lists (multi encoder) and the validity mask as ints
+  std::vector<int>& h = e->h_tgt;
+  h.assign(static_cast<size_t>(n) + 2 * static_cast<size_t>(n) * B, 0);
+  int* counts = h.data();
+  int* lists = counts + n;
+  int* valid = lists + static_cast<size_t>(n) * B;
+  for (int b = 0; b < B; ++b)
+    for (int j = 0; j < n; ++j)
+      if (valid_host[static_cast<size_t>(b) * n + j]) {
+        valid[static_cast<size_t>(b) * n + j] = 1;
+        lists[static_cast<size_t>(j) * B + counts[j]++] = b;
+      }
+  CUDA_TRY(cudaMemcpyAsync(e->tgt_idx, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, s));
+  const int* d_counts = e->tgt_idx;
+  const int* d_lists = e->tgt_idx + n;
+  const int* d_valid = e->tgt_idx + n + static_cast<size_t>(n) * B;
+  const std::vector<TgtStage> st = target_stages(e->cfg);
+  if (type == B200MDM_TARGET_MULTI) {
+    // e_j = L2_j(SiLU(L1_j(target[b, j]))) for the samples whose row j is valid: one group per row, its own sample list
+    int max_rows = 0;
+    for (int j = 0; j < n; ++j) max_rows = counts[j] > max_rows ? counts[j] : max_rows;
+    if (max_rows > 0) {
+      for (int k = 0; k < 2; ++k) {
+        TgtLinear p{};
+        p.x = k == 0 ? target_cond_dev : e->tgt_ha;
+        p.x_gs = k == 0 ? 3 : static_cast<long long>(B) * d;
+        p.ldx = k == 0 ? 3 * n : d;
+        p.w = e->tgt_w[k]; p.w_gs = static_cast<long long>(st[k].N) * st[k].K;
+        p.bias = e->tgt_b[k]; p.b_gs = st[k].N;
+        p.y = k == 0 ? e->tgt_ha : e->tgt_hb; p.y_gs = static_cast<long long>(B) * d; p.ldy = d;
+        p.rows = d_lists; p.counts = d_counts; p.rows_gs = B;
+        p.R = B; p.N = st[k].N; p.K = st[k].K; p.silu_in = k;
+        TRY(launch_tgt_linear(e, p, n, max_rows, s));
+      }
+    }
+    tgt_weighted_sum_kernel<<<B, 128, 0, s>>>(e->tgt_hb, e->tgt_wn, d_valid, e->tgt_out, B, n, d);
+    CUDA_TRY(cudaGetLastError());
+    e->launches++;
+  } else {
+    // single: one MLP on [target | valid].view(B, 4n); split: n MLPs side by side, row j reads columns 4j..4j+3 of the
+    // same input and owns output columns j*d/n .. (j+1)*d/n
+    tgt_input_kernel<<<(B * n * 4 + 255) / 256, 256, 0, s>>>(target_cond_dev, d_valid, e->tgt_x0, B, n);
+    CUDA_TRY(cudaGetLastError());
+    e->launches++;
+    const bool split = type == B200MDM_TARGET_SPLIT;
+    const float* x = e->tgt_x0;
+    for (size_t k = 0; k < st.size(); ++k) {
+      float* y = k + 1 == st.size() ? e->tgt_out : (k % 2 == 0 ? e->tgt_ha : e->tgt_hb);
+      TgtLinear p{};
+      p.x = x;
+      p.x_gs = split ? (k == 0 ? 4 : st[k].K) : 0;
+      p.ldx = k == 0 ? 4 * n : d;
+      p.w = e->tgt_w[k]; p.w_gs = static_cast<long long>(st[k].N) * st[k].K;
+      p.bias = e->tgt_b[k]; p.b_gs = st[k].N;
+      p.y = y; p.y_gs = split ? st[k].N : 0; p.ldy = d;
+      p.R = B; p.N = st[k].N; p.K = st[k].K; p.silu_in = k > 0 ? 1 : 0;
+      TRY(launch_tgt_linear(e, p, st[k].groups, B, s));
+      x = y;
+    }
+  }
+  e->tgt_batch = B;
+  e->tgt_pending = true;
+  return B200MDM_OK;
+}
+
+// The target embedding b200mdm_set_target left for this set_cond* call (nullptr: none); it is consumed either way.
+static int take_target(b200mdm_engine* e, int batch, const float** tgt) {
+  *tgt = nullptr;
+  if (!e->tgt_pending) return B200MDM_OK;
+  e->tgt_pending = false;
+  if (e->tgt_batch != batch)
+    return fail(B200MDM_EINVAL, "b200mdm_set_target was called for batch %d, the conditioning is for batch %d", e->tgt_batch, batch);
+  *tgt = e->tgt_out;
+  return B200MDM_OK;
+}
+
 extern "C" int b200mdm_set_cond(b200mdm_engine* e, int32_t batch, int32_t nframes, const float* cond_embed_dev,
                                 const int64_t* lengths_host, const float* scale_dev, int32_t force_uncond,
                                 const int64_t* action_host, void* stream) {
   if (!e) return fail(B200MDM_EINVAL, "null engine");
   if (e->dec) return fail(B200MDM_EINVAL, "trans_dec engines take their conditioning through b200mdm_set_cond_dec");
+  const float* tgt = nullptr;
+  TRY(take_target(e, batch, &tgt));
   if (!e->finalized) return fail(B200MDM_ESTATE, "weights not finalised");
   if (batch <= 0 || nframes <= 0) return fail(B200MDM_EINVAL, "bad batch / nframes");
   if (nframes + 1 > e->cfg.pos_embed_max_len) return fail(B200MDM_EINVAL, "sequence longer than the positional table");
@@ -919,7 +1137,7 @@ extern "C" int b200mdm_set_cond(b200mdm_engine* e, int32_t batch, int32_t nframe
     e->launches++;
   }
   condproj_fill_kernel<<<e->Bp, 128, 0, s>>>(e->condproj, e->proj, e->b_txt, e->act_emb, e->action, B, d, e->Bp,
-                                             (halves == 1 && force_uncond) ? 1 : 0, e->cfg.cond_mode);
+                                             (halves == 1 && force_uncond) ? 1 : 0, e->cfg.cond_mode, tgt);
   CUDA_TRY(cudaGetLastError());
   e->launches++;
   e->cond_set = true;
@@ -932,6 +1150,8 @@ extern "C" int b200mdm_set_cond_dec(b200mdm_engine* e, int32_t batch, int32_t nf
                                     const float* scale_dev, int32_t force_uncond, void* stream) {
   if (!e) return fail(B200MDM_EINVAL, "null engine");
   if (!e->dec) return fail(B200MDM_EINVAL, "b200mdm_set_cond_dec is for trans_dec engines");
+  const float* tgt = nullptr;
+  TRY(take_target(e, batch, &tgt));
   if (!e->finalized) return fail(B200MDM_ESTATE, "weights not finalised");
   if (batch <= 0 || nframes <= 0 || n_tokens <= 0 || n_tokens > 64) return fail(B200MDM_EINVAL, "bad batch / nframes / n_tokens (1..64)");
   if (nframes + e->ctx > e->cfg.pos_embed_max_len) return fail(B200MDM_EINVAL, "sequence longer than the positional table");
@@ -979,7 +1199,8 @@ extern "C" int b200mdm_set_cond_dec(b200mdm_engine* e, int32_t batch, int32_t nf
   const size_t warps = static_cast<size_t>(B) * Mt * d;
   small_linear_kernel<0><<<static_cast<int>((warps * 32 + 255) / 256), 256, 0, s>>>(e->encperm, e->w_txt, e->b_txt, e->memtok, B * Mt, d, C, C);
   CUDA_TRY(cudaGetLastError());
-  memproj_fill_kernel<<<dim3(Mt, Bp), 128, 0, s>>>(e->memproj, e->memtok, e->b_txt, B, Mt, d, Bp, (halves == 1 && force_uncond) ? 1 : 0);
+  memproj_fill_kernel<<<dim3(Mt, Bp), 128, 0, s>>>(e->memproj, e->memtok, e->b_txt, B, Mt, d, Bp, (halves == 1 && force_uncond) ? 1 : 0,
+                                                   tgt);
   CUDA_TRY(cudaGetLastError());
   e->launches += 3;
   e->cond_set = true;

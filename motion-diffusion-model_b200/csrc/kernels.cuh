@@ -245,10 +245,13 @@ __global__ void small_linear_kernel(const float* __restrict__ x, const float* __
 //   text  : cond = (W clip + b) already in proj[B, d];  uncond = bias          (mask_cond zeros => bias only)
 //   action: cond = action_embedding[a[b]];              uncond = 0             (model/mdm.py:225-227)
 //   none  : 0
+// tgt (optional, [B, d]): the target-location embedding of b200mdm_set_target, added to every row of both halves after
+// the masking (the reference adds it to time_emb, mdm.py:199; (text + target) + time here instead of text + (time +
+// target): only the fp32 association differs).  nullptr: the rows are exactly the above.
 __global__ void condproj_fill_kernel(float* __restrict__ condproj, const float* __restrict__ proj,
                                      const float* __restrict__ bias, const float* __restrict__ action_emb,
                                      const int* __restrict__ action, int B, int d, int rows, int first_uncond,
-                                     int cond_mode) {
+                                     int cond_mode, const float* __restrict__ tgt) {
   const int bp = blockIdx.x;
   if (bp >= rows) return;
   const bool unc = first_uncond ? true : (bp >= B);
@@ -257,6 +260,7 @@ __global__ void condproj_fill_kernel(float* __restrict__ condproj, const float* 
     float v = 0.f;
     if (cond_mode == 1) v = unc ? bias[c] : proj[static_cast<size_t>(b) * d + c];
     else if (cond_mode == 2) v = unc ? 0.f : action_emb[static_cast<size_t>(action[b]) * d + c];
+    if (tgt != nullptr) v += tgt[static_cast<size_t>(b) * d + c];
     condproj[static_cast<size_t>(bp) * d + c] = v;
   }
 }
@@ -298,14 +302,19 @@ __global__ void mem_build_kernel(__half* __restrict__ mem16, const float* __rest
 }
 
 // memproj rows of the packed batch: cond half = W enc + b (already in proj [B*Mt, d], row (b, m)), uncond half = b.
+// tgt (optional, [B, d]): target-location embedding added to every token row of both halves (see condproj_fill_kernel).
 __global__ void memproj_fill_kernel(float* __restrict__ memproj, const float* __restrict__ proj,
-                                    const float* __restrict__ bias, int B, int Mt, int d, int rows_bp, int first_uncond) {
+                                    const float* __restrict__ bias, int B, int Mt, int d, int rows_bp, int first_uncond,
+                                    const float* __restrict__ tgt) {
   const int m = blockIdx.x, bp = blockIdx.y;
   if (bp >= rows_bp) return;
   const bool unc = first_uncond ? true : (bp >= B);
   const int b = bp % B;
-  for (int c = threadIdx.x; c < d; c += blockDim.x)
-    memproj[(static_cast<size_t>(bp) * Mt + m) * d + c] = unc ? bias[c] : proj[(static_cast<size_t>(b) * Mt + m) * d + c];
+  for (int c = threadIdx.x; c < d; c += blockDim.x) {
+    float v = unc ? bias[c] : proj[(static_cast<size_t>(b) * Mt + m) * d + c];
+    if (tgt != nullptr) v += tgt[static_cast<size_t>(b) * d + c];
+    memproj[(static_cast<size_t>(bp) * Mt + m) * d + c] = v;
+  }
 }
 
 // enc_text [Mt, B, C] (reference layout, model/mdm.py:185) -> [B*Mt, C] rows (b, m) so that one small GEMM projects it

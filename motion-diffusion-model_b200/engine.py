@@ -21,11 +21,28 @@ def _stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+def target_validity(rows, target_joint_names, is_heading):
+    """The validity mask EmbedTarget*.forward builds (model/mdm.py:411-416): uint8 [B, n], 1 at row(name) for every name
+    in target_joint_names[b] and at row('heading') when is_heading[b].  target_joint_names: a list of name lists or the
+    object ndarray sample_goal returns (empty sets allowed); an unknown name raises ValueError like the reference's
+    list.index."""
+    heading = np.asarray(torch.as_tensor(is_heading).detach().cpu()).reshape(-1).astype(bool)
+    if len(target_joint_names) != heading.shape[0]:
+        raise ValueError("target_joint_names has %d entries, is_heading %d" % (len(target_joint_names), heading.shape[0]))
+    valid = np.zeros((heading.shape[0], len(rows)), dtype=np.uint8)
+    for b, names in enumerate(target_joint_names):
+        names = [str(j) for j in np.asarray(names, dtype=object).reshape(-1)] + (["heading"] if heading[b] else [])
+        for j in names:
+            valid[b, rows.index(j)] = 1
+    return valid
+
+
 class Engine:
     """One engine per model instance (weights + workspace live on the current CUDA device)."""
 
     def __init__(self, *, arch, latent_dim, ff_size, num_layers, num_heads, njoints, nfeats, cond_mode, cond_dim,
-                 num_actions, mask_frames, pos_embed_max_len, temb_rows, context_len=0):
+                 num_actions, mask_frames, pos_embed_max_len, temb_rows, context_len=0, target_encoder=None,
+                 target_rows=None, target_enc_layers=1):
         self.lib = _lib.load()
         if not torch.cuda.is_available():
             raise RuntimeError("b200mdm needs a CUDA device (sm_100a); there is no CPU fallback")
@@ -33,7 +50,10 @@ class Engine:
         self.cfg = _lib.Config(arch=_lib.ARCH[arch], latent_dim=latent_dim, ff_size=ff_size, num_layers=num_layers,
                                num_heads=num_heads, njoints=njoints, nfeats=nfeats, cond_mode=cm, cond_dim=cond_dim,
                                num_actions=num_actions, mask_frames=int(bool(mask_frames)),
-                               pos_embed_max_len=pos_embed_max_len, temb_rows=temb_rows, context_len=context_len)
+                               pos_embed_max_len=pos_embed_max_len, temb_rows=temb_rows, context_len=context_len,
+                               target_encoder=_lib.TARGET[target_encoder], n_goal_rows=len(target_rows or ()),
+                               target_enc_layers=target_enc_layers)
+        self.target_rows = list(target_rows) if target_encoder is not None else None
         self.dec = arch == "trans_dec"
         self.context_len = context_len
         h = ctypes.c_void_p()
@@ -79,8 +99,35 @@ class Engine:
         self._sched_key = key
 
     # ------------------------------------------------------------------ conditioning
+    def set_target(self, batch, y, device):
+        """y['target_cond'] [B, n, 3] (+ y['target_joint_names'], y['is_heading']) -> b200mdm_set_target, for the next
+        set_cond*.  No 'target_cond' key, or y['target_uncond'] (mask_cond zeros the embedding, model/mdm.py:199): the
+        target is cleared, and the loop is exactly the one without targets.  The target is the same for both halves of a
+        CFG pair (the reference's guidance wrapper deep-copies y, targets included)."""
+        if self.target_rows is None:
+            if y is not None and "target_cond" in y:
+                raise AttributeError("y['target_cond'] given to a model without target conditioning: 'MDM' object has "
+                                     "no attribute 'embed_target_cond' (create it with multi_target_cond=True)")
+            return
+        tc = y.get("target_cond") if y is not None else None
+        if tc is None or bool(y.get("target_uncond", False)):
+            check(self.lib.b200mdm_set_target(self.h, batch, None, None, _stream()))
+            self._keep.pop("target", None)
+            return
+        names, heading = y["target_joint_names"], y["is_heading"]      # KeyError, as the reference's y[...]
+        n = len(self.target_rows)
+        tc = torch.as_tensor(tc).detach().to(device=device, dtype=torch.float32).contiguous()
+        if tuple(tc.shape) != (batch, n, 3):
+            raise ValueError("y['target_cond'] must be [batch, %d, 3] (rows %s), got %s" % (n, self.target_rows, tuple(tc.shape)))
+        valid = target_validity(self.target_rows, names, heading)
+        if valid.shape[0] != batch:
+            raise ValueError("target_joint_names / is_heading describe %d samples, the batch has %d" % (valid.shape[0], batch))
+        check(self.lib.b200mdm_set_target(self.h, batch, _ptr(tc), valid.ctypes.data_as(ctypes.c_void_p), _stream()))
+        self._keep["target"] = (tc, valid)
+
     def set_cond(self, batch, nframes, y, guided, device):
         """Canonicalise model_kwargs['y'] (data_loaders/tensors.py:22-64 schema).  `guided` => CFG pair."""
+        self.set_target(batch, y, device)
         text_embed = y.get("text_embed") if y is not None else None
         if self.dec:
             return self._set_cond_dec(batch, nframes, y, guided, device)

@@ -7,9 +7,11 @@ It uploads them once into the B200 engine (fp16 repack) and calls `b200mdm_denoi
 
 Implemented: arch='trans_enc' with cond_mode in {no_cond, text (CLIP features), action}; arch='trans_dec' with
 text_encoder_type='bert' (DiP: BERT token memory, prefix completion, model/mdm.py:203-206,255-270); hml_vec / rot6d /
-xyz data_rep.
-Not implemented (raise): arch 'gru', data_rep 'rot_vel', multi-target conditioning (CLoSD), emb_trans_dec,
-emb_policy != 'add', trans_dec with CLIP features.
+xyz data_rep; target-location conditioning (multi_target_cond, the CLoSD "DiP with target conditioning" checkpoint:
+y['target_cond'] / y['target_joint_names'] / y['is_heading'], model/mdm.py:197-199) with the single, multi and split
+target encoders.
+Not implemented (raise): arch 'gru', data_rep 'rot_vel', emb_trans_dec, emb_policy != 'add', trans_dec with CLIP
+features.
 """
 import numpy as np
 import torch
@@ -43,6 +45,35 @@ class _Bag(nn.Module):
         if head not in self._modules:
             self.add_module(head, _Bag())
         self._modules[head].add(rest, tensor, buffer)
+
+
+def target_row_names(all_goal_joint_names):
+    """The rows of y['target_cond']: EmbedTarget*.extended_goal_joint_names (model/mdm.py:402,425,453)."""
+    return list(all_goal_joint_names) + ["traj", "heading"]
+
+
+def _target_spec(encoder, d, layers, rows):
+    """embed_target_cond.* keys of EmbedTargetLocSingle / Multi / Split (model/mdm.py:399-480, utils/misc.py:5-9)."""
+    n = len(rows)
+    p = "embed_target_cond."
+    if encoder == "single":
+        s = [(p + "mlp.0.weight", (d, 4 * n), "lin"), (p + "mlp.0.bias", (d,), "lin")]
+        for l in range(1, layers + 1):
+            s += [(p + "mlp.%d.weight" % (2 * l), (d, d), "lin"), (p + "mlp.%d.bias" % (2 * l), (d,), "lin")]
+        return s
+    if encoder == "split":
+        ds = d // n
+        s = []
+        for j in range(n):
+            s += [(p + "mini_mlps.%d.0.weight" % j, (ds, 4), "lin"), (p + "mini_mlps.%d.0.bias" % j, (ds,), "lin")]
+            for l in range(1, layers + 1):
+                s += [(p + "mini_mlps.%d.%d.weight" % (j, 2 * l), (ds, ds), "lin"), (p + "mini_mlps.%d.%d.bias" % (j, 2 * l), (ds,), "lin")]
+        return s
+    s = []
+    for name in rows:
+        q = p + "target_loc_emb.%s." % name
+        s += [(q + "0.weight", (d, 3), "lin"), (q + "0.bias", (d,), "lin"), (q + "2.weight", (d, d), "lin"), (q + "2.bias", (d,), "lin")]
+    return s + [(p + "target_all_loc_emb.weights", (n,), "normal")]
 
 
 def _spec(arch, d, ff, layers, input_feats, cond_mode, cond_dim, num_actions):
@@ -107,6 +138,8 @@ class MDM(_Bag):
         self.is_prefix_comp = self.total_len > 0
         self.all_goal_joint_names = kargs.get("all_goal_joint_names", [])
         self.multi_target_cond = kargs.get("multi_target_cond", False)
+        self.multi_encoder_type = kargs.get("multi_encoder_type", "multi")
+        self.target_enc_layers = kargs.get("target_enc_layers", 1)
         self.text_encoder_type = kargs.get("text_encoder_type", "clip")
         self.pos_embed_max_len = kargs.get("pos_embed_max_len", 5000)
         self.temb_rows = min(self.pos_embed_max_len, kargs.get("num_model_timesteps", 1000))
@@ -118,8 +151,15 @@ class MDM(_Bag):
                                       "an ablation and out of scope" % (arch,))
         if activation != "gelu":
             raise NotImplementedError("the fused FFN epilogue implements exact GELU only (model_util.py:63)")
-        if data_rep == "rot_vel" or self.multi_target_cond or self.emb_policy != "add":
-            raise NotImplementedError("rot_vel / multi-target / emb_policy='cat' variants are outside the hot path")
+        if data_rep == "rot_vel" or self.emb_policy != "add":
+            raise NotImplementedError("rot_vel / emb_policy='cat' variants are outside the hot path")
+        self.target_rows = target_row_names(self.all_goal_joint_names) if self.multi_target_cond else None
+        if self.multi_target_cond:
+            if self.multi_encoder_type not in ("single", "multi", "split"):
+                raise NotImplementedError("multi_encoder_type=%r: the single, multi and split target encoders are "
+                                          "implemented (model/mdm.py:67-73)" % (self.multi_encoder_type,))
+            if self.multi_encoder_type == "split" and latent_dim % len(self.target_rows):
+                raise AssertionError("split target encoder needs latent_dim %% %d == 0 (model/mdm.py:430)" % len(self.target_rows))
         if arch == "trans_enc":
             if self.is_prefix_comp:
                 raise NotImplementedError("prefix completion is implemented for arch='trans_dec' (DiP) only")
@@ -134,6 +174,9 @@ class MDM(_Bag):
         for key, shape, kind in _spec(arch, latent_dim, ff_size, num_layers, self.input_feats, self.cond_mode,
                                       self.clip_dim, num_actions):
             self.add(key, _init(shape, kind))
+        if self.multi_target_cond:
+            for key, shape, kind in _target_spec(self.multi_encoder_type, latent_dim, self.target_enc_layers, self.target_rows):
+                self.add(key, _init(shape, kind))
         self.add("sequence_pos_encoder.pe", positional_table(self.pos_embed_max_len, latent_dim).unsqueeze(1), buffer=True)
         self._engine = None
         self._engine_dirty = True
@@ -186,16 +229,30 @@ class MDM(_Bag):
                                       nfeats=self.nfeats, cond_mode=self.cond_mode, cond_dim=self.clip_dim,
                                       num_actions=max(1, self.num_actions), mask_frames=self.mask_frames,
                                       pos_embed_max_len=self.pos_embed_max_len, temb_rows=self.temb_rows,
-                                      context_len=self.context_len if self.arch == "trans_dec" else 0)
+                                      context_len=self.context_len if self.arch == "trans_dec" else 0,
+                                      target_encoder=self.multi_encoder_type if self.multi_target_cond else None,
+                                      target_rows=self.target_rows, target_enc_layers=self.target_enc_layers)
             self._engine_device = dev
             self._engine_dirty = True
         if self._engine_dirty:
-            sd = {k: v for k, v in self.state_dict().items()}
-            sd["sequence_pos_encoder.pe"] = self.sequence_pos_encoder.pe.squeeze(1)
+            sd = self.engine_state_dict()
             with torch.cuda.device(dev):
                 self._engine.load_state_dict(sd)
             self._engine_dirty = False
         return self._engine
+
+    def engine_state_dict(self):
+        """The tensors b200mdm_load_weight receives: the state_dict plus the positional table, with the multi target
+        encoder's per-joint MLPs renamed from joint name to row index (the C side addresses rows; only the host knows
+        all_goal_joint_names)."""
+        sd = {k: v for k, v in self.state_dict().items()}
+        if self.multi_target_cond and self.multi_encoder_type == "multi":
+            pre = "embed_target_cond.target_loc_emb."
+            for j, name in enumerate(self.target_rows):
+                for suffix in ("0.weight", "0.bias", "2.weight", "2.bias"):
+                    sd["%s%d.%s" % (pre, j, suffix)] = sd.pop("%s%s.%s" % (pre, name, suffix))
+        sd["sequence_pos_encoder.pe"] = self.sequence_pos_encoder.pe.squeeze(1)
+        return sd
 
     def forward(self, x, timesteps, y=None):
         """x [B, njoints, nfeats, T] fp32, timesteps [B] (model timesteps), y dict -> [B, njoints, nfeats, T]

@@ -14,6 +14,7 @@ its slice from its own torch stream (rank-dependent results).
 
 One process per GPU, ``torch.distributed`` (backend nccl on GPUs; the same code runs on gloo/CPU in the tests).
 """
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -60,7 +61,8 @@ def gather_objects(obj, group=None):
     return out
 
 
-_BATCH_KEYS = ("mask", "lengths", "scale", "action", "inpainting_mask", "inpainted_motion", "prefix")
+_BATCH_KEYS = ("mask", "lengths", "scale", "action", "inpainting_mask", "inpainted_motion", "prefix", "target_cond",
+               "is_heading")
 
 
 def shard_model_kwargs(model_kwargs, lo, hi):
@@ -77,6 +79,8 @@ def shard_model_kwargs(model_kwargs, lo, hi):
             out[k] = v[lo:hi].contiguous()
         elif k in ("text", "tokens") and isinstance(v, (list, tuple)):
             out[k] = list(v[lo:hi])
+        elif k == "target_joint_names" and isinstance(v, (list, tuple, np.ndarray)):   # a name set per sample
+            out[k] = v[lo:hi] if isinstance(v, np.ndarray) else list(v[lo:hi])
         else:
             out[k] = v
     return {**model_kwargs, "y": out}

@@ -21,8 +21,69 @@ def _normal(rng, shape, std):
     return torch.from_numpy((rng.standard_normal(size=shape) * std).astype(np.float32))
 
 
+HML_GOAL_ROWS = ["pelvis", "left_foot", "right_foot", "left_wrist", "right_wrist", "head", "traj", "heading"]
+
+
 def synthetic_state_dict(arch="trans_enc", latent_dim=512, ff_size=1024, num_layers=8, input_feats=263,
-                         cond_dim=512, cond_mode="text", num_actions=1, seed=0):
+                         cond_dim=512, cond_mode="text", num_actions=1, seed=0, target_encoder=None, target_enc_layers=1,
+                         n_goal_rows=8):
+    """target_encoder ('single' / 'multi' / 'split'): also the embed_target_cond.* keys of a multi_target_cond model
+    (humanml rows: HML_GOAL_ROWS; n_goal_rows = 2 keeps 'traj' and 'heading' only).  They come from a stream of their
+    own, so the other tensors are the same as without them."""
+    sd = _base_state_dict(arch, latent_dim, ff_size, num_layers, input_feats, cond_dim, cond_mode, num_actions, seed)
+    if target_encoder is not None:
+        sd.update(_target_state_dict(target_encoder, latent_dim, target_enc_layers, n_goal_rows, seed))
+    return sd
+
+
+def _target_state_dict(encoder, d, layers, n, seed):
+    """At the reference's default init the target moves a trans_enc output by only ~0.5 %; the last layer here is
+    scaled up so that it moves it by several per cent (a missing target shows far outside the parity tolerance), and
+    the multi encoder's row weights are positive so that their sum stays away from 0."""
+    if n > len(HML_GOAL_ROWS) or n < 2:
+        raise ValueError("n_goal_rows must be 2..%d" % len(HML_GOAL_ROWS))
+    rows = HML_GOAL_ROWS[: n - 2] + ["traj", "heading"]
+    rng = np.random.default_rng(seed + 7001)
+    sd = {}
+    gain = 6.0
+
+    def linear(prefix, out_f, in_f, g=1.0):
+        b = 1.0 / math.sqrt(in_f)
+        sd[prefix + ".weight"] = _uniform(rng, (out_f, in_f), b * g)
+        sd[prefix + ".bias"] = _uniform(rng, (out_f,), b * g)
+
+    p = "embed_target_cond."
+    if encoder == "single":
+        linear(p + "mlp.0", d, 4 * n)
+        for l in range(1, layers + 1):
+            linear(p + "mlp.%d" % (2 * l), d, d, gain if l == layers else 1.0)
+    elif encoder == "split":
+        ds = d // n
+        for j in range(n):
+            linear(p + "mini_mlps.%d.0" % j, ds, 4)
+            for l in range(1, layers + 1):
+                linear(p + "mini_mlps.%d.%d" % (j, 2 * l), ds, ds, gain if l == layers else 1.0)
+    elif encoder == "multi":
+        for name in rows:
+            linear(p + "target_loc_emb.%s.0" % name, d, 3)
+            linear(p + "target_loc_emb.%s.2" % name, d, d, gain)
+        sd[p + "target_all_loc_emb.weights"] = torch.from_numpy(rng.uniform(0.5, 1.5, size=n).astype(np.float32))
+    else:
+        raise ValueError("unsupported target encoder %r" % (encoder,))
+    return sd
+
+
+def synthetic_targets(batch, joint_sets, heading, n_goal_rows=8, seed=17):
+    """y['target_cond'] [B, n, 3] (every row filled, valid or not -- the single and split encoders read them all),
+    y['target_joint_names'] (the given per-sample name lists) and y['is_heading'] (bool [B])."""
+    rng = np.random.default_rng(seed)
+    tc = torch.from_numpy(rng.standard_normal((batch, n_goal_rows, 3)).astype(np.float32))
+    assert len(joint_sets) == batch and len(heading) == batch
+    return dict(target_cond=tc, target_joint_names=[list(s) for s in joint_sets],
+                is_heading=torch.tensor([bool(h) for h in heading]))
+
+
+def _base_state_dict(arch, latent_dim, ff_size, num_layers, input_feats, cond_dim, cond_mode, num_actions, seed):
     rng = np.random.default_rng(seed)
     d = latent_dim
     sd = {}
